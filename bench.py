@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Harmony hot path (cluster() + moe_correct_ridge() to convergence).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 Metric (BASELINE.json): cells/sec to convergence of the full Harmony loop.
 A *step* = one complete run of the loop from the post-upload state: restore Z_cos, the
@@ -21,6 +21,10 @@ computed once, untimed, on a 100k-cell subsample; both arms start from the same 
 Workloads (BASELINE.json configs): syn1m (default; 1M cells x 50 PCs x 20 batches, K=100,
 per GPU -- weak scaling), syn10m8 (10M x 50 x 50 batches over 8 GPUs => 1.25M per GPU),
 syn5m8 (5M x 50, covariates 30+4, K=200 over 8 GPUs => 625k per GPU).
+
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs) so that two builds can be compared
+output for output: the inputs, initial centroids included, depend only on the arguments.  The device's reductions
+are not bitwise reproducible, so two runs of one build differ in the last bits (compare with a tolerance).
 """
 import argparse
 import json
@@ -40,6 +44,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True              # the benchmark leaves the tree as it found it (it may be read-only)
 
 WORKLOADS = {
     "syn1m": dict(per_gpu=1_000_000, d=50, levels=[20], K=100,
@@ -52,6 +57,7 @@ WORKLOADS = {
 }
 SEED = 0
 INIT_SUBSAMPLE = 100_000
+DUMP_SAMPLE_BYTES = 48 << 20      # --dump-outputs: Z_corr + R rows of the cell sample; the other outputs are small
 
 
 def algorithmic_bytes(d, K, V):
@@ -118,13 +124,17 @@ class ClockSampler:
 
 def init_centroids(w, N_total, seed=SEED):
     """k-means++ / 25 Lloyd iterations (the reference's sklearn settings, harmony.py:370-371)
-    on the unit-normalised first INIT_SUBSAMPLE cells.  Untimed; identical for both arms."""
+    on the unit-normalised first INIT_SUBSAMPLE cells.  Untimed; identical for both arms.
+    One thread: sklearn's multi-threaded Lloyd reduces its partial sums in scheduling order, so its
+    centroids differ in the last bits from run to run, and with them every later result."""
     from sklearn.cluster import KMeans
+    from threadpoolctl import threadpool_limits
     from harmonypy_b200.synthetic import make_synthetic_arrays
     n = min(N_total, INIT_SUBSAMPLE)
     Z, _ = make_synthetic_arrays(N_total, w["d"], w["levels"], seed=seed, lo=0, hi=n)
     Zc = Z / np.linalg.norm(Z, axis=1, keepdims=True)
-    km = KMeans(n_clusters=w["K"], init="k-means++", n_init=1, max_iter=25, random_state=seed).fit(Zc)
+    with threadpool_limits(limits=1):
+        km = KMeans(n_clusters=w["K"], init="k-means++", n_init=1, max_iter=25, random_state=seed).fit(Zc)
     return km.cluster_centers_.astype(np.float32)
 
 
@@ -181,13 +191,6 @@ def _oracle_run(w, Y0, n_sample):
 def load_reference():
     """The UNMODIFIED reference package staged under baseline/_ref (baseline/stage_reference.py), or None."""
     ref_dir = os.path.join(ROOT, "baseline", "_ref")
-    if not os.path.exists(os.path.join(ref_dir, "harmonypy", "harmony.py")):
-        try:
-            sys.path.insert(0, os.path.join(ROOT, "baseline"))
-            import stage_reference
-            stage_reference.stage(verbose=False)
-        except Exception:
-            pass
     if not os.path.exists(os.path.join(ref_dir, "harmonypy", "harmony.py")):
         return None
     if ref_dir not in sys.path:
@@ -335,6 +338,25 @@ def golden_parity(device_index, comm=None):
     return out
 
 
+def dump_outputs(out_dir, ho):
+    """What the timed path returned in its last step, one DIR/<name>.npy each, under 64 MB in all: Z_corr and R on
+    one fixed, seeded sample of this rank's cells in cell order (DUMP_SAMPLE_BYTES for the two), the centroids Y,
+    O and E in full (float32); the objectives and kmeans_rounds (float64)."""
+    from harmonypy_b200 import _cabi
+    os.makedirs(out_dir, exist_ok=True)
+    Zc = ho.result_local()
+    n_local = Zc.shape[0]
+    n = min(n_local, DUMP_SAMPLE_BYTES // (4 * (ho.d + ho.K)))
+    cells = np.sort(np.random.default_rng(SEED).choice(n_local, n, replace=False))
+    arrays = {"Z_corr": Zc[cells], "R": ho._engine.get(_cabi.R)[cells], "Y": ho.Y, "O": ho.O, "E": ho.E}
+    arrays = {k: np.asarray(v, dtype=np.float32) for k, v in arrays.items()}
+    for name in ("objective_harmony", "objective_kmeans", "objective_kmeans_dist", "objective_kmeans_entropy",
+                 "objective_kmeans_cross", "kmeans_rounds"):
+        arrays[name] = np.asarray(getattr(ho, name), dtype=np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 def run_ours(args, w):
     import torch
@@ -400,6 +422,8 @@ def run_ours(args, w):
         e1.record(stream)
         barrier()
     ms_total = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ho)
     if dist is not None:
         t = torch.tensor([ms_total], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -534,7 +558,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--engine-opt", action="append", default=[], help="name=int engine option (debug / A-B runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (rank 0's cells)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     w = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, w)

@@ -3,6 +3,8 @@ include/harmony_b200.h declares, and refuses to run without a GPU (no silent CPU
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -41,12 +43,17 @@ def test_version_string(lib):
 
 
 def test_create_fails_loudly_without_gpu(lib):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from harmonypy_b200 import _cabi
-    with pytest.raises(_cabi.EngineError, match="hmy_create"):
-        _cabi.Engine(0, 100, 100, 0, 10, 8, [2])
+    """A child process that sees no CUDA device (hidden from it where the machine has one) cannot create an engine."""
+    code = ("from harmonypy_b200 import _cabi\n"
+            "try:\n"
+            "    _cabi.Engine(0, 100, 100, 0, 10, 8, [2])\n"
+            "except _cabi.EngineError as e:\n"
+            "    assert 'hmy_create' in str(e), e\n"
+            "else:\n"
+            "    raise SystemExit('an engine was created without a CUDA device')\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
 
 
 def test_create_validates_arguments(lib):

@@ -56,24 +56,24 @@ def test_simpson_edge_cases_follow_the_reference():
     assert np.isfinite(s).all() and (s > 0).all()
 
 
-REF = "/root/reference"
+RANDOM_CASES = [(600, 3, 30, 0), (900, 20, 15, 1), (500, 8, 42, 2)]
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "harmonypy", "lisi.py")),
-                    reason="the reference checkout is only present in the build container")
-@pytest.mark.parametrize("n,d,perp,seed", [(600, 3, 30, 0), (900, 20, 15, 1), (500, 8, 42, 2)])
-def test_oracle_equals_live_reference_on_random_data(n, d, perp, seed):
-    import sys
-    sys.dont_write_bytecode = True
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    from harmonypy.lisi import compute_lisi as ref_lisi
+def _random_problem(n, d, seed):
     rng = np.random.default_rng(seed)
     t = rng.integers(0, 4, n)
     X = rng.normal(size=(4, d))[t] * 2.5 + rng.normal(size=(n, d))
     meta = pd.DataFrame({"type": pd.Categorical(t.astype(str)), "batch": pd.Categorical(rng.integers(0, 3, n).astype(str)),
                          "one": pd.Categorical(["a"] * n)})
-    want = ref_lisi(X, meta, ["type", "batch", "one"], perp)
+    return X, meta
+
+
+@pytest.mark.parametrize("n,d,perp,seed", RANDOM_CASES)
+def test_oracle_equals_live_reference_on_random_data(n, d, perp, seed):
+    """Against what the unmodified reference's compute_lisi returned on the same seeded data
+    (tests/golden/make_golden_random.py)."""
+    X, meta = _random_problem(n, d, seed)
+    want = np.load(os.path.join(GOLDEN, "random_lisi.npz"))[f"seed{seed}_lisi"]
     got = compute_lisi(X, meta, ["type", "batch", "one"], perp)
     np.testing.assert_allclose(got, want, rtol=1e-9)
     np.testing.assert_allclose(got[:, 2], 1.0, rtol=1e-12)          # a single category: LISI = 1 everywhere

@@ -1,34 +1,29 @@
-"""Differential test of the CPU oracle against the LIVE reference over randomised configurations.
+"""Differential test of the CPU oracle against the reference over randomised configurations.
 
-The committed golden fixtures pin the oracle on three datasets; this test widens the pin across the argument space
-(per-covariate / per-level theta and lambda, dynamic lambda, tau, sigma, block sizes, 1-3 covariates, small K) by
-running the reference itself -- its fp64 restatement, i.e. harmonypy/harmony.py with float32 -> float64 substituted in a
-temp copy exactly as tests/golden/make_golden.py does -- and the fp64 oracle on the same inputs, the same sklearn
-centroids and the same permutation stream.  Agreement is at rounding level (1e-9), not at fp32 noise level.
-
-Runs only where /root/reference exists (the build container); skipped on the GPU box.  CPU only.
+The golden fixtures of the three datasets pin the oracle there; this test widens the pin across the argument space
+(per-covariate / per-level theta and lambda, dynamic lambda, tau, sigma, block sizes, 1-3 covariates, small K).  It
+runs the fp64 oracle on seeded random problems and compares with what the reference's fp64 restatement (harmonypy/
+harmony.py with float32 -> float64 substituted, as tests/golden/make_golden.py does) returned on the same inputs,
+the same sklearn centroids and the same permutation stream: tests/golden/random_oracle.npz, written by
+tests/golden/make_golden_random.py.  Agreement is at rounding level (1e-9), not at fp32 noise level.  CPU only.
 """
+import hashlib
 import os
-import sys
 
 import numpy as np
 import pandas as pd
 import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "harmonypy", "harmony.py")),
-                                reason="the reference checkout is only present in the build container")
-
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 @pytest.fixture(scope="module")
 def ref64():
-    sys.dont_write_bytecode = True
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    import make_golden
-    return make_golden, make_golden.load_reference_module(True)
+    return np.load(os.path.join(GOLDEN, "random_oracle.npz"))
+
+
+def _digest(a):
+    return hashlib.sha1(np.ascontiguousarray(a).tobytes()).hexdigest()[:16]
 
 
 def _problem(rng, N, d, levels):
@@ -57,32 +52,36 @@ CASES = [
 
 @pytest.mark.parametrize("case", range(len(CASES)))
 def test_oracle_fp64_equals_live_reference_fp64(ref64, case):
-    from oracle.harmony_oracle import HarmonyOracle, onehot_from_codes
-    make_golden, mod64 = ref64
-    N, d, levels, kw = CASES[case]
+    from oracle.harmony_oracle import HarmonyOracle, onehot_from_codes, torch_perm_source
+    g = {k[len(f"c{case}_"):]: ref64[k] for k in ref64.files if k.startswith(f"c{case}_")}
+    N, d, levels, _ = CASES[case]                   # the keyword arguments went to the reference's run_harmony
     rng = np.random.default_rng(100 + case)
     Z, meta = _problem(rng, N, d, levels)
-    kw = dict(kw, max_iter_harmony=kw.get("max_iter_harmony", 3))
-    stage_cells = np.arange(0, N, 7)
-    # the reference draws its own centroids and permutations; both are captured and replayed into the oracle
-    ho, cap = make_golden.run_captured(mod64, pd.DataFrame(Z.astype(np.float64)), meta, list(meta.columns), kw, stage_cells)
+    assert _digest(Z) == str(g["Z_digest"]), "the seeded input is not the one the reference ran on"
 
     codes = np.stack([pd.Categorical(meta[v]).codes for v in meta.columns]).astype(np.int32)
     lv = np.array([len(pd.Categorical(meta[v]).categories) for v in meta.columns], dtype=np.int32)
     phi = onehot_from_codes(codes, lv, np.float64)
-    assert np.array_equal(phi, ho.Phi.T)
-    orc = HarmonyOracle(Z.astype(np.float64).T, phi, ho.Pr_b, ho.sigma, ho.theta, ho.lamb, alpha=float(ho.alpha),
-                        lambda_estimation=bool(ho.lambda_estimation), block_size=float(ho.block_size),
-                        epsilon_kmeans=float(ho.epsilon_kmeans), epsilon_harmony=float(ho.epsilon_harmony),
-                        max_iter_kmeans=int(ho.max_iter_kmeans), dtype=np.float64)
-    perms = iter(cap["perms"])
-    orc.init_from_centroids(np.asarray(cap["Y0"], dtype=np.float64).T)
-    orc.harmonize(int(ho.max_iter_harmony), lambda: next(perms))
+    assert _digest(phi.astype(np.uint8)) == str(g["Phi_digest"])
+    orc = HarmonyOracle(Z.astype(np.float64).T, phi, g["Pr_b"], g["sigma"], g["theta"], g["lamb"], alpha=float(g["alpha"]),
+                        lambda_estimation=bool(g["lambda_estimation"]), block_size=float(g["block_size"]),
+                        epsilon_kmeans=float(g["epsilon_kmeans"]), epsilon_harmony=float(g["epsilon_harmony"]),
+                        max_iter_kmeans=int(g["max_iter_kmeans"]), dtype=np.float64)
+    # the reference's centroids and its permutation stream (torch.manual_seed(0), one randperm per update_R)
+    src, want_perms = torch_perm_source(N, 0), iter(g["perm_digests"])
 
-    assert list(orc.kmeans_rounds) == list(ho.kmeans_rounds)
-    scale = np.abs(ho.Z_corr).max()
-    assert np.abs(orc.Z_corr.T - ho.Z_corr).max() / scale < 1e-9
-    np.testing.assert_allclose(orc.objective_harmony, ho.objective_harmony, rtol=1e-10)
-    np.testing.assert_allclose(orc.objective_kmeans, ho.objective_kmeans, rtol=1e-10)
-    np.testing.assert_allclose(orc.R.T, ho.R, atol=1e-11)
-    np.testing.assert_allclose(orc.O, ho.O, rtol=1e-9, atol=1e-10)
+    def perms():
+        p = src()
+        assert _digest(p.astype(np.int64)) == str(next(want_perms)), "permutation stream differs from the reference's"
+        return p
+    orc.init_from_centroids(np.asarray(g["Y0"], dtype=np.float64).T)
+    orc.harmonize(int(g["max_iter_harmony"]), perms)
+
+    assert list(orc.kmeans_rounds) == list(g["kmeans_rounds"])
+    assert next(want_perms, None) is None
+    zs, rs = int(ref64["zcorr_step"]), int(ref64["r_step"])
+    assert np.abs(orc.Z_corr.T[::zs] - g["Zcorr_sub"]).max() / float(g["Zcorr_absmax"]) < 1e-9
+    np.testing.assert_allclose(orc.objective_harmony, g["objective_harmony"], rtol=1e-10)
+    np.testing.assert_allclose(orc.objective_kmeans, g["objective_kmeans"], rtol=1e-10)
+    np.testing.assert_allclose(orc.R.T[::rs], g["R_sub"], atol=1e-11)
+    np.testing.assert_allclose(orc.O, g["O"], rtol=1e-9, atol=1e-10)
