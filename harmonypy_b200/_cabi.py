@@ -42,6 +42,7 @@ SYMBOLS = {
     "hmy_counter": (C.c_int64, [C.c_void_p, C.c_char_p]),
     "hmy_timer_ms": (C.c_double, [C.c_void_p, C.c_char_p]),
     "hmy_set_allreduce": (C.c_int, [C.c_void_p, ALLREDUCE_FN, C.c_void_p]),
+    "hmy_set_rank": (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     "hmy_comm_export": (C.c_int, [C.c_void_p, C.c_void_p]),
     "hmy_comm_attach": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "hmy_lisi_compute": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_double, C.c_void_p]),
@@ -210,7 +211,9 @@ class Engine:
         return obj[0], obj[1], obj[2]
 
     def kmeans_init(self, seed, max_iter=25, tol=1e-4):
-        """k-means++ / Lloyd on the resident Z_cos (hmy_kmeans_init).  Returns (K x d means, info dict)."""
+        """k-means++ / Lloyd on the resident Z_cos (hmy_kmeans_init).  Returns (K x d means, info dict).
+        On a shard of the cells (n_local < n_global) it is collective: every rank calls it with the same arguments,
+        after set_allreduce and set_rank, and every rank gets the same result."""
         Y = np.empty((self.K, self.d), dtype=np.float32)
         info = (C.c_double * 3)()
         self._ck(self.lib.hmy_kmeans_init(self.h, C.c_uint64(int(seed) & (2**64 - 1)), int(max_iter), float(tol), _ptr(Y), info),
@@ -287,6 +290,10 @@ class Engine:
         blob = b"".join(handles)
         assert len(blob) == 64 * world
         self._ck(self.lib.hmy_comm_attach(self.h, int(rank), int(world), blob), "hmy_comm_attach")
+
+    def set_rank(self, rank, world):
+        """This rank's place among `world` ranks (hmy_set_rank): needed by kmeans_init on a shard of the cells."""
+        self._ck(self.lib.hmy_set_rank(self.h, int(rank), int(world)), "hmy_set_rank")
 
     def set_allreduce(self, pyfunc):
         """pyfunc(dev_ptr:int, count:int, dtype:int, stream:int) -> 0 on success."""

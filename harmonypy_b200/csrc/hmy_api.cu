@@ -100,6 +100,8 @@ struct hmy_ctx {
     std::vector<void*> xopened;                            // peers' buffers opened through IPC
     bool fused = false, force_fused_kernel = false;
     unsigned int xseq = 0;
+    int rank = -1, world = 0;                              // hmy_set_rank / hmy_comm_attach (host side only)
+    double* kmi_agree = nullptr; int kmi_agree_world = 0;  // [world][HMY_KMI_AGREE] checks exchanged by hmy_kmeans_init
 };
 
 #define CK(call)                                                                                   \
@@ -894,11 +896,163 @@ extern "C" int hmy_init_from_centroids(hmy_ctx* ctx, const float* Y0, double obj
 }
 
 // ---- optional: k-means++ / Lloyd initialisation on the device (hmy_kmeans_init.cuh) -----------
+
+// Per-rank record of the exchange that precedes the first collective of a sharded initialisation:
+// ok, K, d, n_global, cell_offset, n_local, max_iter, tol, seed >> 32, seed & 0xFFFFFFFF (all exact in fp64).
+#define HMY_KMI_AGREE 10
+
+static int record_rank(hmy_ctx* ctx, int rank, int world) {
+    if (world > ctx->kmi_agree_world) {
+        if (dev_alloc(ctx, &ctx->kmi_agree, (size_t)world * HMY_KMI_AGREE)) return 1;
+        ctx->kmi_agree_world = world;
+    }
+    ctx->rank = rank; ctx->world = world;
+    return 0;
+}
+
+// Cells sharded over ranks (n_local < n_global).  Every collective below is entered by every rank the same number of
+// times: the only decisions between them are taken from all-reduced data (identical on every rank) or from checks whose
+// inputs are identical on every rank.  A rank that stopped alone would leave the others waiting in a collective.
+static int kmeans_init_sharded(hmy_ctx* ctx, uint64_t seed, int max_iter, double tol, float* Y_host, double info[3]) {
+    HmyDev& st = ctx->st;
+    if (!ctx->ar) FAIL("hmy_kmeans_init: the context holds a shard of the cells (n_local < n_global) and needs the sum "
+                       "all-reduce over ranks: call hmy_set_allreduce first");
+    if (ctx->rank < 0) FAIL("hmy_kmeans_init: the context holds a shard of the cells (n_local < n_global) and needs its "
+                            "rank: call hmy_set_rank (or hmy_comm_attach) first");
+    // checks that depend on the global shape only: the same outcome on every rank, so they may fail before any collective
+    const int K = st.K, dp = st.dp, S = 2 + dp, W = ctx->world, R = ctx->rank;
+    if (st.Nglobal < K) FAIL("hmy_kmeans_init: fewer cells than clusters");
+    if (st.Nglobal > (1LL << 32)) FAIL("hmy_kmeans_init: sharded initialisation supports at most 2^32 cells");
+    const size_t smem_lloyd = ((size_t)K * (dp | 1) + K + (size_t)K * dp + (size_t)(HMY_KMI_THREADS / 32) * dp) * sizeof(float) + (size_t)K * sizeof(unsigned int);
+    if (smem_lloyd > 200 * 1024) FAIL("hmy_kmeans_init: K * d too large for the shared-memory Lloyd kernel (K (2 d + 2) floats <= 200 KB)");
+    const size_t nS = (size_t)K * dp, nT = nS + K + 1;            // Lloyd table [sums K dp | counts K | inertia]
+    // checks and allocations of this rank: their outcome is exchanged before the first collective that depends on them
+    std::string local_err;
+    if (!ctx->have_data) local_err = "hmy_kmeans_init: upload the data first";
+    else if (!Y_host) local_err = "hmy_kmeans_init: NULL output";
+    else if (max_iter < 0 || !(tol >= 0.0)) local_err = "hmy_kmeans_init: max_iter and tol must be non-negative";
+    float *mind2 = nullptr, *C = nullptr; unsigned long long* best = nullptr; unsigned int* counts = nullptr;
+    double *slots = nullptr, *tab = nullptr, *scal = nullptr; int* fail = nullptr;
+    std::vector<void*> tmp;
+    auto cleanup = [&]() { for (void* p : tmp) cudaFree(p); };
+    auto dev = [&](void** p, size_t bytes) {
+        if (!local_err.empty()) return;
+        const cudaError_t e = cudaMalloc(p, bytes);
+        if (e == cudaSuccess) { tmp.push_back(*p); return; }
+        cudaGetLastError();
+        local_err = std::string("hmy_kmeans_init: cudaMalloc failed: ") + cudaGetErrorString(e);
+    };
+    dev((void**)&mind2, (size_t)st.N * sizeof(float));
+    dev((void**)&C, nS * sizeof(float));
+    dev((void**)&best, (size_t)K * sizeof(unsigned long long));
+    dev((void**)&counts, (size_t)K * sizeof(unsigned int));
+    dev((void**)&slots, (size_t)W * S * sizeof(double));
+    dev((void**)&tab, nT * sizeof(double));
+    dev((void**)&scal, 4 * sizeof(double));
+    dev((void**)&fail, sizeof(int));
+    if (local_err.empty()) {
+        const cudaError_t e = cudaFuncSetAttribute((const void*)k_lloyd_assign, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_lloyd);
+        if (e != cudaSuccess) { cudaGetLastError(); local_err = std::string("hmy_kmeans_init: ") + cudaGetErrorString(e); }
+    }
+#define KCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { cleanup(); char b_[512]; snprintf(b_, sizeof b_, "hmy_kmeans_init: %s failed: %s", #call, cudaGetErrorString(e_)); ctx->err = b_; return 1; } } while (0)
+#define KAR(p, n) do { if (allreduce(ctx, (p), (int64_t)(n), 1)) { cleanup(); return 1; } } while (0)
+    // every rank's checks, arguments and cell range, gathered exactly (one slot per rank, zeros elsewhere)
+    {
+        std::vector<double> ag((size_t)W * HMY_KMI_AGREE, 0.0);
+        double* a = ag.data() + (size_t)R * HMY_KMI_AGREE;
+        const double mine[HMY_KMI_AGREE] = {local_err.empty() ? 1.0 : 0.0, (double)K, (double)st.d, (double)st.Nglobal,
+                                            (double)st.cell_offset, (double)st.N, (double)max_iter, tol >= 0.0 ? tol : -1.0,
+                                            (double)(seed >> 32), (double)(seed & 0xFFFFFFFFull)};
+        std::copy(mine, mine + HMY_KMI_AGREE, a);
+        KCK(cudaMemcpyAsync(ctx->kmi_agree, ag.data(), ag.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        KAR(ctx->kmi_agree, ag.size());
+        KCK(cudaMemcpyAsync(ag.data(), ctx->kmi_agree, ag.size() * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        KCK(cudaStreamSynchronize(ctx->stream));
+        if (!local_err.empty()) { cleanup(); FAIL(local_err); }
+        std::vector<std::pair<double, double>> ranges;
+        for (int r = 0; r < W; ++r) {
+            const double* o = ag.data() + (size_t)r * HMY_KMI_AGREE;
+            if (o[0] != 1.0) { cleanup(); ctx->err = "hmy_kmeans_init: rank " + std::to_string(r) + " failed its checks (see its error)"; return 1; }
+            for (int i = 1; i < HMY_KMI_AGREE; ++i)
+                if (i != 4 && i != 5 && o[i] != mine[i]) {
+                    cleanup(); FAIL("hmy_kmeans_init: the ranks disagree on K, d, n_global, seed, max_iter or tol");
+                }
+            ranges.emplace_back(o[4], o[5]);
+        }
+        std::sort(ranges.begin(), ranges.end());
+        double next = 0.0;
+        for (auto& rg : ranges) { if (rg.first != next) break; next += rg.second; }
+        if (next != (double)st.Nglobal) { cleanup(); FAIL("hmy_kmeans_init: the ranks' cell ranges do not cover the n_global cells exactly once"); }
+    }
+    // seeding: one slot exchange per centre, no host synchronisation until the end
+    KCK(cudaMemsetAsync(best, 0xFF, (size_t)K * sizeof(unsigned long long), ctx->stream));
+    KCK(cudaMemsetAsync(C, 0, nS * sizeof(float), ctx->stream));
+    KCK(cudaMemsetAsync(fail, 0, sizeof(int), ctx->stream));
+    const long long first_id = (long long)(hmy_splitmix64((unsigned long long)seed) % (unsigned long long)st.Nglobal);
+    const unsigned int grid = (unsigned int)std::min<long long>(4LL * ctx->sms, (st.N + (HMY_KMI_THREADS / 32) - 1) / (HMY_KMI_THREADS / 32));
+    for (int c = 0; c < K; ++c) {
+        if (c > 0) {
+            k_kmpp_pass_sharded<<<grid, HMY_KMI_THREADS, dp * sizeof(float), ctx->stream>>>(st, C, c, (unsigned long long)seed, mind2, best);
+            ctx->launches++;
+        }
+        k_kmpp_publish<<<1, 256, 0, ctx->stream>>>(st, best, c, first_id, R, W, slots);
+        KCK(cudaGetLastError());
+        KAR(slots, (size_t)W * S);
+        k_kmpp_pick<<<1, 64, 0, ctx->stream>>>(slots, W, dp, c, C, fail);
+        ctx->launches += 2;
+    }
+    KCK(cudaGetLastError());
+    {
+        int hfail = 0;
+        KCK(cudaMemcpyAsync(&hfail, fail, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+        KCK(cudaStreamSynchronize(ctx->stream));
+        if (hfail) { cleanup(); FAIL("hmy_kmeans_init: fewer distinct cells than clusters"); }   // the same on every rank
+    }
+    // Lloyd: one all-reduce of the table, one of the "another iteration" votes; the loop runs while any rank votes for it
+    double h[4] = {0.0, 0.0, 0.0, 0.0};   // squared shift | mean feature variance | votes | inertia
+    int iters = 0;
+    for (int it = 0; it < max_iter; ++it) {
+        KCK(cudaMemsetAsync(tab, 0, nT * sizeof(double), ctx->stream));
+        KCK(cudaMemsetAsync(counts, 0, (size_t)K * sizeof(unsigned int), ctx->stream));
+        k_lloyd_assign<<<grid, HMY_KMI_THREADS, smem_lloyd, ctx->stream>>>(st, C, tab, counts, tab + nS + K);
+        k_lloyd_pack_counts<<<1, 256, 0, ctx->stream>>>(counts, K, tab + nS);
+        KCK(cudaGetLastError());
+        KAR(tab, nT);
+        k_lloyd_update_global<<<1, 256, 0, ctx->stream>>>(st, C, tab, tol, scal);
+        KCK(cudaGetLastError());
+        KAR(scal + 2, 1);
+        ctx->launches += 3;
+        KCK(cudaMemcpyAsync(h, scal, 4 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        KCK(cudaStreamSynchronize(ctx->stream));
+        iters = it + 1;
+        if (h[2] == 0.0) break;
+    }
+    // rank 0's centres and info to everyone
+    {
+        const double tail[3] = {(double)iters, h[3], h[0]};
+        const double none[3] = {0.0, 0.0, 0.0};
+        k_kmi_share<<<(unsigned int)((nS + 255) / 256), 256, 0, ctx->stream>>>(C, nS, R == 0, tab);
+        ctx->launches++;
+        KCK(cudaGetLastError());
+        KCK(cudaMemcpyAsync(tab + nS, R == 0 ? tail : none, 3 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        KAR(tab, nS + 3);
+        std::vector<double> out(nS + 3);
+        KCK(cudaMemcpyAsync(out.data(), tab, out.size() * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        KCK(cudaStreamSynchronize(ctx->stream));
+        for (int k = 0; k < K; ++k) for (int j = 0; j < st.d; ++j) Y_host[(size_t)k * st.d + j] = (float)out[(size_t)k * dp + j];
+        if (info) { info[0] = out[nS]; info[1] = out[nS + 1]; info[2] = out[nS + 2]; }
+    }
+    cleanup();
+#undef KAR
+#undef KCK
+    return 0;
+}
+
 extern "C" int hmy_kmeans_init(hmy_ctx* ctx, uint64_t seed, int max_iter, double tol, float* Y_host, double info[3]) {
     HmyDev& st = ctx->st;
     CK(cudaSetDevice(ctx->device));
+    if (st.N < st.Nglobal) return kmeans_init_sharded(ctx, seed, max_iter, tol, Y_host, info);
     if (!ctx->have_data) FAIL("hmy_kmeans_init: upload the data first");
-    if (st.Nglobal != st.N) FAIL("hmy_kmeans_init: single-GPU contexts only (with cells sharded over ranks pass init_centroids)");
     if (!Y_host) FAIL("hmy_kmeans_init: NULL output");
     if (max_iter < 0 || !(tol >= 0.0)) FAIL("hmy_kmeans_init: max_iter and tol must be non-negative");
     if (st.N < st.K) FAIL("hmy_kmeans_init: fewer cells than clusters");
@@ -1351,5 +1505,11 @@ extern "C" int hmy_comm_attach(hmy_ctx* ctx, int rank, int world, const void* al
     }
     st.xrank = rank; st.xworld = world;
     ctx->fused = world > 1;
-    return 0;
+    return record_rank(ctx, rank, world);
+}
+
+extern "C" int hmy_set_rank(hmy_ctx* ctx, int rank, int world) {
+    CK(cudaSetDevice(ctx->device));
+    if (world < 1 || rank < 0 || rank >= world) FAIL("hmy_set_rank: need 0 <= rank < world");
+    return record_rank(ctx, rank, world);
 }

@@ -4,7 +4,7 @@
 // stream, so the parity configurations keep sklearn; what it is compared with is oracle/kmeans_init_oracle.py, the
 // same algorithm in NumPy with the same counter-based random numbers.
 //
-// STATUS: written at the end of round 1 without GPU time left; compiled only, GPU tests opt-in (HMY_TEST_KMINIT=1).
+// Runs with the plain GPU suite (tests/test_gpu_kmeans_init.py, tests/test_gpu_dist_kmeans_init.py).
 //
 // Seeding (k-means++, Arthur & Vassilvitskii): centre 0 uniformly; centre c with probability proportional to the
 // squared distance to the nearest centre so far.  The draw is an exponential race, argmin_i E_i / D2_i with
@@ -12,6 +12,14 @@
 // in memory (the engine stores them sorted by covariate combination).  Lloyd: one warp per cell, lanes over clusters,
 // per-CTA shared-memory sums, fp64 global sums; stops at sklearn's criterion (squared centre shift <=
 // tol * mean feature variance) or after max_iter iterations.
+//
+// Cells sharded over ranks: because the race keys depend on the global cell id only, every rank runs the pass over its
+// own cells (k_kmpp_pass_sharded, the previous centre read from the gathered centre table) and publishes its winner as
+// one slot {key, global id, row} of a world x (2 + dp) fp64 table whose other slots are zero (k_kmpp_publish); a sum
+// all-reduce of that table is an exact all-gather (fp32 values and ids are exact in fp64, x + 0 = x), and
+// k_kmpp_pick takes the minimum by (key, global id) -- the cell a single GPU holding every cell picks.  Lloyd keeps
+// k_lloyd_assign; its local sums, counts and inertia travel as one fp64 table through one all-reduce, and
+// k_lloyd_update_global divides by the global cell count.
 #pragma once
 #include "hmy_common.cuh"
 
@@ -127,20 +135,22 @@ __global__ void __launch_bounds__(HMY_KMI_THREADS) k_lloyd_assign(HmyDev st, con
     if (lane == 0 && my_inertia != 0.0) atomicAdd(inertia, my_inertia);
 }
 
-// new centres = means (an empty cluster keeps its centre); info[0] = squared shift, info[1] = mean feature variance
-__global__ void k_lloyd_update(HmyDev st, float* C, const double* sums, const unsigned int* counts, double* info) {
+// new centres = means (an empty cluster keeps its centre); info[0] = squared shift, info[1] = mean feature variance.
+// n_cells: the number of cells the sums run over (all ranks' cells when the sums are global).
+template <class CountT>
+__device__ void lloyd_update(const HmyDev& st, float* C, const double* sums, const CountT* counts, double n_cells, double* info) {
     __shared__ double s_shift[32], s_mean2[32];
     const int K = st.K, dp = st.dp, d = st.d, tid = threadIdx.x;
     double shift = 0.0, mean2 = 0.0;
     for (int j = tid; j < d; j += blockDim.x) {                           // ||mean of all cells||^2, one feature per thread
         double s = 0.0;
         for (int k = 0; k < K; ++k) s += sums[(size_t)k * dp + j];
-        s /= (double)st.N;
+        s /= n_cells;
         mean2 += s * s;
     }
     for (int i = tid; i < K * dp; i += blockDim.x) {
         const int k = i / dp, j = i - k * dp;
-        if (j < d && counts[k] > 0u) {
+        if (j < d && counts[k] > (CountT)0) {
             const float nc = (float)(sums[i] / (double)counts[k]);
             const double df = (double)nc - (double)C[i];
             shift += df * df;
@@ -156,6 +166,114 @@ __global__ void k_lloyd_update(HmyDev st, float* C, const double* sums, const un
         info[0] = a;
         info[1] = (1.0 - b) / (double)d;                                  // rows of Z_cos have unit length: E|z|^2 = 1
     }
+}
+
+__global__ void k_lloyd_update(HmyDev st, float* C, const double* sums, const unsigned int* counts, double* info) {
+    lloyd_update(st, C, sums, counts, (double)st.N, info);
+}
+
+// ---- cells sharded over ranks ----------------------------------------------------------------------------------------
+
+// One seeding step on this rank's cells: D2 to centre c - 1 (row c - 1 of the gathered centres C), running minimum, race
+// for centre c.  best[c] must be ~0ull on entry; afterwards it is {key bits, global id} of the local winner.
+__global__ void __launch_bounds__(HMY_KMI_THREADS) k_kmpp_pass_sharded(HmyDev st, const float* C, int c, unsigned long long seed,
+                                                                       float* mind2, unsigned long long* best) {
+    extern __shared__ __align__(16) unsigned char kmi_smem[];
+    float* sy = reinterpret_cast<float*>(kmi_smem);                       // [dp] the newest centre
+    __shared__ unsigned long long s_best[HMY_KMI_THREADS / 32];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, dp = st.dp;
+    for (int j = tid; j < dp; j += HMY_KMI_THREADS) sy[j] = C[(size_t)(c - 1) * dp + j];
+    __syncthreads();
+    unsigned long long mine = ~0ull;
+    const long long nw = (long long)gridDim.x * (HMY_KMI_THREADS / 32);
+    for (long long pos = (long long)blockIdx.x * (HMY_KMI_THREADS / 32) + warp; pos < st.N; pos += nw) {
+        const float* z = st.Zcos + (size_t)pos * dp;
+        float s = 0.f;
+        for (int j = lane; j < dp; j += 32) { const float u = z[j] - sy[j]; s = fmaf(u, u, s); }
+        s = warp_sum(s);
+        if (lane == 0) {
+            const float m = (c == 1) ? s : fminf(mind2[pos], s);
+            mind2[pos] = m;
+            if (m > 0.f) {
+                const unsigned long long id = (unsigned long long)(st.cell_offset + st.order[pos]);   // < 2^32 (host check)
+                const float key = (float)(-log(hmy_kmi_uniform(seed, c, id)) / (double)m);
+                const unsigned long long packed = ((unsigned long long)__float_as_uint(key) << 32) | id;
+                mine = packed < mine ? packed : mine;
+            }
+        }
+    }
+    if (lane == 0) s_best[warp] = mine;
+    __syncthreads();
+    if (tid == 0) {
+        unsigned long long b = s_best[0];
+        for (int w = 1; w < HMY_KMI_THREADS / 32; ++w) b = s_best[w] < b ? s_best[w] : b;
+        if (b != ~0ull) atomicMin(&best[c], b);
+    }
+}
+
+// This rank's candidate for centre c as slot `rank` of slots [world][2 + dp] = {key, global id, row}; every other slot
+// is zeroed, so that the sum over ranks gathers all candidates exactly.  Centre 0 is cell first_id (key 0) on the rank
+// that holds it; a rank without a candidate publishes key = +inf.
+__global__ void k_kmpp_publish(HmyDev st, const unsigned long long* best, int c, long long first_id, int rank, int world,
+                               double* slots) {
+    const int dp = st.dp, S = 2 + dp;
+    long long id = -1;
+    double key = 0.0;
+    if (c == 0) {
+        if (first_id >= st.cell_offset && first_id < st.cell_offset + st.N) id = first_id;
+    } else if (best[c] != ~0ull) {
+        id = (long long)(best[c] & 0xFFFFFFFFull);
+        key = (double)__uint_as_float((unsigned int)(best[c] >> 32));
+    }
+    const float* row = (id >= 0) ? st.Zcos + (size_t)st.pos_of[id - st.cell_offset] * dp : nullptr;
+    for (int i = threadIdx.x; i < world * S; i += blockDim.x) {
+        const int w = i / S, j = i - w * S;
+        double v = 0.0;
+        if (w == rank) v = (j == 0) ? (id >= 0 ? key : INFINITY) : (id < 0) ? 0.0 : (j == 1) ? (double)id : (double)row[j - 2];
+        slots[i] = v;
+    }
+}
+
+// Row c of the centres = the gathered candidate with the least (key, global id); *fail = 1 when no rank had one (no cell
+// at a positive distance from the centres so far).
+__global__ void k_kmpp_pick(const double* slots, int world, int dp, int c, float* C, int* fail) {
+    __shared__ int s_w;
+    const int S = 2 + dp;
+    if (threadIdx.x == 0) {
+        int bw = -1;
+        for (int w = 0; w < world; ++w) {
+            const double k = slots[(size_t)w * S], id = slots[(size_t)w * S + 1];
+            if (!(k < INFINITY)) continue;
+            if (bw < 0 || k < slots[(size_t)bw * S] || (k == slots[(size_t)bw * S] && id < slots[(size_t)bw * S + 1])) bw = w;
+        }
+        s_w = bw;
+        if (bw < 0) *fail = 1;
+    }
+    __syncthreads();
+    if (s_w < 0) return;
+    for (int j = threadIdx.x; j < dp; j += blockDim.x) C[(size_t)c * dp + j] = (float)slots[(size_t)s_w * S + 2 + j];
+}
+
+// counts [K] -> the fp64 slice of the Lloyd table [sums K dp | counts K | inertia] that is summed over ranks
+__global__ void k_lloyd_pack_counts(const unsigned int* counts, int K, double* tab_counts) {
+    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < K; k += gridDim.x * blockDim.x) tab_counts[k] = (double)counts[k];
+}
+
+// k_lloyd_update on the table summed over ranks.  info: [0] squared shift, [1] mean feature variance, [2] 1 if this rank
+// would run another iteration (shift^2 > tol * variance), else 0, [3] global inertia.
+__global__ void k_lloyd_update_global(HmyDev st, float* C, const double* tab, double tol, double* info) {
+    const size_t nS = (size_t)st.K * st.dp;
+    lloyd_update(st, C, tab, tab + nS, (double)st.Nglobal, info);
+    if (threadIdx.x == 0) {
+        info[2] = (info[0] <= tol * info[1]) ? 0.0 : 1.0;
+        info[3] = tab[nS + st.K];
+    }
+}
+
+// rank 0's centres (fp32 -> fp64), zeros on the other ranks: the sum over ranks hands everyone rank 0's centres exactly
+__global__ void k_kmi_share(const float* C, size_t n, int keep, double* out) {
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+        out[i] = keep ? (double)C[i] : 0.0;
 }
 
 #endif  // HMY_NONTEMPLATE_KERNELS

@@ -250,6 +250,7 @@ def _cuda_engine_factory(problem, lo, hi, device_index, comm, options):
         torch.cuda.set_device(device_index)
         eng.set_stream(torch.cuda.current_stream().cuda_stream)
         eng.set_allreduce(comm.allreduce_devptr)
+        eng.set_rank(comm.rank, comm.world)
     return eng
 
 
@@ -277,7 +278,9 @@ def run_harmony(data_mat, meta_data, vars_use, theta=None, lamb=None, sigma=0.1,
         Where the k-means initialisation of harmony.py:369-373 runs when ``init_centroids`` is not given.
         "sklearn" (default): exactly the reference's call.  "device": k-means++ / Lloyd on the GPU
         (``hmy_kmeans_init``; same algorithm, its own random stream keyed by ``random_state``) -- for sizes
-        where sklearn dominates the wall time; single GPU only.
+        where sklearn dominates the wall time.  With ``comm`` every rank initialises from its own cells (also
+        pre-sharded input, where no rank holds all cells): the ranks exchange one slot per k-means++ step and the
+        Lloyd sums, pick exactly the seeds one GPU holding all cells would, and all start from the same centroids.
     """
     problem, vars_use = prepare_problem(data_mat, meta_data, vars_use, theta, lamb, sigma, nclust, tau)
     dev = get_device(device)
@@ -500,10 +503,9 @@ class Harmony:
 
     def init_cluster(self, random_state, init_centroids=None):
         """harmony.py:366-392.  k-means++ / Lloyd initialisation stays with sklearn on the host
-        exactly as in the reference; everything after it runs on the device."""
+        exactly as in the reference (or runs on the device with init_mode="device"; with sharded cells
+        that call is collective: every rank makes it); everything after it runs on the device."""
         if init_centroids is None and self.init_mode == "device":
-            if self.comm is not None and self.comm.world > 1:
-                raise ValueError("init_mode='device' runs on one GPU; with sharded cells pass init_centroids")
             if self.verbose:
                 logger.info("Computing initial centroids on the device (k-means++ / Lloyd)...")
             init_centroids, self.kmeans_init_info = self._engine.kmeans_init(int(random_state), max_iter=25, tol=1e-4)
@@ -511,7 +513,8 @@ class Harmony:
             if self.comm is None or self.comm.rank == 0:
                 from sklearn.cluster import KMeans
                 if self.problem.shard_lo is not None:
-                    raise ValueError("pre-sharded input needs init_centroids (no rank holds all cells)")
+                    raise ValueError("pre-sharded input needs init_centroids or init_mode='device' "
+                                     "(no rank holds all cells)")
                 Z = self.problem.Z
                 Z_cos = Z / np.linalg.norm(Z, axis=1, keepdims=True)
                 if self.verbose:

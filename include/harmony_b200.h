@@ -94,9 +94,19 @@ int hmy_init_from_centroids(hmy_ctx* ctx, const float* Y0_host_Kxd, double obj[3
  * n_init=1, max_iter=25) on the unit-length cells) for sizes where it dominates the wall time: k-means++
  * seeding and Lloyd iterations on the resident Z_cos, stopped by sklearn's criterion (squared centre shift <=
  * tol * mean feature variance) or after max_iter iterations.  It cannot reproduce sklearn's random stream:
- * parity configurations keep sklearn and pass the centroids to hmy_init_from_centroids.  Single-GPU contexts.
+ * parity configurations keep sklearn and pass the centroids to hmy_init_from_centroids.
  * Y_host: K x d means (feed them to hmy_init_from_centroids); info: iterations run, inertia of the last
- * assignment pass, last squared centre shift (may be NULL). */
+ * assignment pass, last squared centre shift (may be NULL).
+ *
+ * Cells sharded over ranks (n_local < n_global): a COLLECTIVE call -- every rank calls it with the same seed, max_iter
+ * and tol, after hmy_set_allreduce and hmy_set_rank (or hmy_comm_attach); it fails before any all-reduce when either is
+ * missing.  The ranks' cell ranges must cover the n_global cells exactly once; n_global >= K is required (a shard may
+ * hold fewer than K cells), n_global <= 2^32.  The seeds are exactly the cells a single GPU holding all cells picks
+ * (the race keys depend on the global cell id only); the Lloyd sums, counts and inertia are summed over ranks.  Every
+ * rank returns the same Y_host and info (rank 0's): global inertia and shift.  Cost: 1 all-reduce of 10 x world
+ * doubles for the checks, K of world x (2 + d') doubles for the seeding (d' = d rounded up to 4), 2 per Lloyd
+ * iteration (K (d' + 1) + 1 doubles and 1 double), 1 of K d' + 3 doubles at the end.  All ranks fail together when any rank's checks or
+ * allocations fail, or when they disagree on K, d, n_global or the arguments. */
 int hmy_kmeans_init(hmy_ctx* ctx, uint64_t seed, int max_iter, double tol, float* Y_host_Kxd, double info[3]);
 
 /* One iteration of the loop body of cluster() (harmony.py:443-453): centroid update,
@@ -163,6 +173,11 @@ double hmy_timer_ms(hmy_ctx* ctx, const char* name);
 
 /* Staged mode: the library calls `fn` wherever a small table must be summed over ranks. */
 int hmy_set_allreduce(hmy_ctx* ctx, hmy_allreduce_fn fn, void* user);
+
+/* This context's rank among `world` ranks (0 <= rank < world), for the collectives of hmy_kmeans_init on sharded cells.
+ * Host-side bookkeeping only: the round kernels and the staged / fused mode do not change.  hmy_comm_attach records
+ * the rank too. */
+int hmy_set_rank(hmy_ctx* ctx, int rank, int world);
 
 /* Fused mode: ranks exchange the small tables inside the persistent round kernel through
  * peer-mapped device memory.  Each rank exports a 64-byte handle of its exchange buffer;
